@@ -3,6 +3,8 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's B200 engine
     python bench.py --impl reference --gpus N --steps K --warmup W   # the reference's CPU path
+    python bench.py ... --dump-outputs DIR    # also save a seeded sample of the last timed step's outputs as .npy, so
+                                              # that two builds can be compared output for output on identical inputs
 
 Workload (config.workload): BASELINE.json configs[1] - r1041_e82_400bps_sup_v5 consensus on a
 synthetic 10 Mb draft: 1111 windows x 10000 pileup columns x 10 features (chunk_len 10000,
@@ -331,6 +333,36 @@ def workload_name(cfg=2):
     return CONFIGS[cfg]["name"]
 
 
+DUMP_BYTES = 48 << 20      # --dump-outputs: probabilities + labels, both as float32 (24 bytes per position)
+
+
+def dump_selection(B, T):
+    """Windows (a fixed seeded sample, sorted) and leading columns per window whose outputs fit in DUMP_BYTES."""
+    cols = min(T, DUMP_BYTES // 24)
+    n = max(1, min(B, DUMP_BYTES // (24 * cols)))
+    return np.sort(np.random.default_rng(0).choice(B, n, replace=False)), cols
+
+
+def copy_outputs(lm, dev, d_probs, d_labels, T, windows, cols):
+    """The sampled part of one step's device outputs ([B,T,5] float32 probabilities, [B,T] uint8 labels) on the host."""
+    lib, ffi = lm.lib, lm.ffi
+    probs = np.empty((len(windows), cols, 5), dtype=np.float32)
+    labels = np.empty((len(windows), cols), dtype=np.uint8)
+    for i, w in enumerate(windows):
+        lm.check(lib.mdk_memcpy_d2h(dev, ffi.from_buffer(probs[i]), ffi.cast("float *", d_probs) + int(w) * T * 5,
+                                    probs[i].nbytes))
+        lm.check(lib.mdk_memcpy_d2h(dev, ffi.from_buffer(labels[i]), ffi.cast("uint8_t *", d_labels) + int(w) * T,
+                                    labels[i].nbytes))
+    return probs, labels
+
+
+def write_outputs(out_dir, probs, labels, windows):
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "probs.npy"), probs)
+    np.save(os.path.join(out_dir, "labels.npy"), labels.astype(np.float32))
+    np.save(os.path.join(out_dir, "windows.npy"), windows.astype(np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -350,7 +382,14 @@ def main():
                     help="columns per window in the CPU sample (0 = the full window length for the cpu_baseline of the "
                          "default run, ~15 s; sized for ~12 s per step for --impl reference)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's probabilities and labels (rank 0, a seeded sample of at most "
+                         "48 MB) and the sampled window indices as DIR/{probs,labels,windows}.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
 
     capture_stdout()
     rank = int(os.environ.get("RANK", "0"))
@@ -476,6 +515,12 @@ def main():
     lm.check(lib.mdk_engine_timer_stop(eng, ms))     # end event after every lane and the copy streams
     barrier()
     clocks = sampler.stop()
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        # copied now: the forwards below write into the same output sets
+        last = (step_no[0] - 1) & 1
+        dump_windows, dump_cols = dump_selection(B, T)
+        dumped = copy_outputs(lm, dev, d_probs_set[last], d_labels_set[last], T, dump_windows, dump_cols)
     dev_ms = float(ms[0])
     launches = model.launch_count() - launches0 + (args.steps if args.config == 5 else 0)
     tm = ffi.new("mdk_timings *")
@@ -651,6 +696,8 @@ def main():
     }
     if args.config == 4:
         line["variant_decode"] = variant_leg(h_probs[(args.steps - 1) % n_slots], B, T, dev)
+    if dumped is not None:
+        write_outputs(args.dump_outputs, *dumped, dump_windows)
     emit(line)
     if dist is not None:
         dist.destroy_process_group()

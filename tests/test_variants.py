@@ -4,7 +4,6 @@ Goldens: tests/golden/variants.npz, written by tests/golden/make_variant_golden.
 medaka.labels.HaploidLabelScheme.decode_variants / medaka.variant.join_samples (with variant_columns compiled from the
 reference's src/medaka_rnn_variants.c), plus the reference's literal cases (medaka/test/test_labels.py:279-399).
 """
-import ctypes
 import json
 import os
 
@@ -126,27 +125,15 @@ def test_oracle_join_matches_reference_golden():
 
 
 def test_reference_c_variant_columns_matches_oracle():
-    """oracle/_ref/libmedaka_rnn_variants.so is the reference's own src/medaka_rnn_variants.c (oracle/Makefile)."""
-    so = os.path.join(ROOT, "oracle", "_ref", "libmedaka_rnn_variants.so")
-    if not os.path.exists(so):
-        pytest.skip("oracle/_ref not built (needs /root/reference: make -C oracle)")
-    lib = ctypes.CDLL(so)
-    lib.variant_columns.argtypes = [ctypes.c_void_p] * 4 + [ctypes.c_size_t]
-    lib.variant_columns.restype = None
-    rs = np.random.RandomState(9)
-    for trial in range(20):
-        n = int(rs.randint(1, 3000))
-        is_minor = rs.uniform(size=n) < 0.3
-        is_minor[0] = False
-        idx = np.arange(n)
-        last_major = np.maximum.accumulate(np.where(~is_minor, idx, -1))
-        minor = np.ascontiguousarray(idx - last_major, dtype=np.uintp)
-        ref = rs.randint(0, 5, n)
-        pred = np.where(rs.uniform(size=n) < 0.85, ref, rs.randint(0, 5, n))
-        r32, p32 = np.ascontiguousarray(ref, dtype=np.int32), np.ascontiguousarray(pred, dtype=np.int32)   # wchar_t
-        out = np.zeros(n, dtype=np.bool_)
-        lib.variant_columns(minor.ctypes.data, r32.ctypes.data, p32.ctypes.data, out.ctypes.data, n)
-        assert np.array_equal(out, labels_oracle.variant_columns(minor.astype(np.int64), ref, pred))
+    """The verdicts of the reference's own src/medaka_rnn_variants.c on 20 seeded pileups, recorded in
+    tests/golden/variant_columns.npz by tests/golden/make_variant_columns_golden.py."""
+    g = np.load(os.path.join(ROOT, "tests", "golden", "variant_columns.npz"))
+    offs = np.concatenate(([0], np.cumsum(g["lengths"])))
+    assert len(g["lengths"]) == 20
+    for a, b in zip(offs[:-1], offs[1:]):
+        minor = g["minor"][a:b].astype(np.int64)
+        ref, pred = g["reference"][a:b].astype(np.int64), g["prediction"][a:b].astype(np.int64)
+        assert np.array_equal(labels_oracle.variant_columns(minor, ref, pred), g["is_var"][a:b])
 
 
 # ------------------------------------------------------------------------------------------------ CUDA path (GPU)
