@@ -79,8 +79,9 @@ struct RlConv1 {
 __global__ void __launch_bounds__(RL_C) rl_embed_conv1_kernel(const int8_t *__restrict__ x, const uint8_t *__restrict__ mask,
                                                               RlConv1 a, int64_t P, int D, int F, int use_dwells,
                                                               float *__restrict__ y1) {
-    // grid: (position chunks of 32, B * D); thread = output channel
-    const int64_t bd = blockIdx.y;
+    // grid: (B * D, position chunks of 32, at most 65 535 of them: a CTA strides over the rest); thread = output channel.
+    // B * D goes in x: 100 reads per window put it past y's limit of 65 535 at 656 windows per call
+    const int64_t bd = blockIdx.x;
     if (!mask[bd]) return;
     const int64_t b = bd / D;
     const int d = (int)(bd % D);
@@ -90,25 +91,27 @@ __global__ void __launch_bounds__(RL_C) rl_embed_conv1_kernel(const int8_t *__re
     for (int i = 0; i < nin; ++i) w[i] = a.w[c * nin + i];
     const float bias = a.b[c], mean = a.bn_mean[c], invstd = a.bn_invstd[c], bw = a.bn_w[c], bb = a.bn_b[c];
     __shared__ float in[32][RL_EMB + 2];
-    const int64_t p0 = (int64_t)blockIdx.x * 32;
-    if (threadIdx.x < 32) {
-        const int64_t p = p0 + threadIdx.x;
-        if (p < P) {
-            const int8_t *v = x + ((b * P + p) * D + d) * F;
-            const int base = min(max((int)v[0], 0), 5), strand = min(max((int)v[2] + 1, 0), 2);
-            for (int i = 0; i < RL_EMB; ++i) in[threadIdx.x][i] = a.emb_base[base * RL_EMB + i] + a.emb_strand[strand * RL_EMB + i];
-            in[threadIdx.x][RL_EMB] = (float)v[1] / 25.0f - 1.0f;
-            if (use_dwells) in[threadIdx.x][RL_EMB + 1] = (float)v[4];
+    for (int64_t p0 = (int64_t)blockIdx.y * 32; p0 < P; p0 += (int64_t)gridDim.y * 32) {
+        __syncthreads();                                       // the previous chunk's rows are consumed
+        if (threadIdx.x < 32) {
+            const int64_t p = p0 + threadIdx.x;
+            if (p < P) {
+                const int8_t *v = x + ((b * P + p) * D + d) * F;
+                const int base = min(max((int)v[0], 0), 5), strand = min(max((int)v[2] + 1, 0), 2);
+                for (int i = 0; i < RL_EMB; ++i) in[threadIdx.x][i] = a.emb_base[base * RL_EMB + i] + a.emb_strand[strand * RL_EMB + i];
+                in[threadIdx.x][RL_EMB] = (float)v[1] / 25.0f - 1.0f;
+                if (use_dwells) in[threadIdx.x][RL_EMB + 1] = (float)v[4];
+            }
         }
-    }
-    __syncthreads();
-    for (int i = 0; i < 32; ++i) {
-        const int64_t p = p0 + i;
-        if (p >= P) break;
-        float acc = bias;
-        for (int k = 0; k < nin; ++k) acc = fmaf(w[k], in[i][k], acc);
-        acc = fmaxf(acc, 0.f);
-        y1[(bd * P + p) * RL_C + c] = (acc - mean) * invstd * bw + bb;
+        __syncthreads();
+        for (int i = 0; i < 32; ++i) {
+            const int64_t p = p0 + i;
+            if (p >= P) break;
+            float acc = bias;
+            for (int k = 0; k < nin; ++k) acc = fmaf(w[k], in[i][k], acc);
+            acc = fmaxf(acc, 0.f);
+            y1[(bd * P + p) * RL_C + c] = (acc - mean) * invstd * bw + bb;
+        }
     }
 }
 
@@ -1042,7 +1045,10 @@ int mdk_rl_forward(mdk_rl_engine *e, const int8_t *x_host, int64_t B, int64_t P,
     MDK_REQUIRE(B >= 1 && P >= 1 && D >= 1, MDK_ERR_ARG, "rl_forward: need B, P, D >= 1");
     MDK_REQUIRE(F == (e->use_dwells ? 5 : 4) || (!e->use_dwells && F >= 4), MDK_ERR_ARG,
                 "rl_forward: feature vector length does not match the model (4, or 5 with dwells)");
-    MDK_REQUIRE(D <= 65535 && B <= 65535, MDK_ERR_ARG, "rl_forward: B, D <= 65535");
+    // grid limits (y, z <= 65 535; x < 2^31): B is gridDim.z of the convolution and y of the pooling, the read groups
+    // gridDim.y (<= 16 384), B * D gridDim.x of the mask and fp32 k = 1 convolution kernels; positions are in x (or
+    // strided over in y)
+    MDK_REQUIRE(D <= 65535 && B <= 65535 && B * D <= 0x7fffffff, MDK_ERR_ARG, "rl_forward: B, D <= 65535, B * D < 2^31");
     MDK_CUDA(cudaSetDevice(e->device));
     int rc = rl_prepare(e);
     if (rc) return rc;
@@ -1078,8 +1084,8 @@ int mdk_rl_forward(mdk_rl_engine *e, const int8_t *x_host, int64_t B, int64_t P,
         rl_conv17_tc_kernel<<<dim3((unsigned)((P + CT_NPOS - 1) / CT_NPOS), (unsigned)n_groups, (unsigned)B), 256, CT_SMEM, s>>>(
             d_x, d_mask, c1, c17, e->c17_tc, P, (int)D, (int)F, e->use_dwells, dgroup, d_part);
     } else {
-        rl_embed_conv1_kernel<<<dim3((unsigned)((P + 31) / 32), (unsigned)(B * D)), RL_C, 0, s>>>(d_x, d_mask, c1, P, (int)D, (int)F,
-                                                                                             e->use_dwells, d_y1);
+        rl_embed_conv1_kernel<<<dim3((unsigned)(B * D), (unsigned)std::min<int64_t>((P + 31) / 32, 65535)), RL_C, 0, s>>>(
+            d_x, d_mask, c1, P, (int)D, (int)F, e->use_dwells, d_y1);
         MDK_CUDA(cudaFuncSetAttribute(rl_conv17_pool_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, RL_CONV_SMEM));
         rl_conv17_pool_kernel<<<dim3((unsigned)((P + RL_PT - 1) / RL_PT), (unsigned)n_groups, (unsigned)B), 256, RL_CONV_SMEM, s>>>(
             d_y1, d_mask, c17, P, (int)D, dgroup, d_part);

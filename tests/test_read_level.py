@@ -13,19 +13,33 @@ GOLD = os.path.join(os.path.dirname(__file__), "golden", "rl_forward.npz")
 TOL = 2e-5
 
 
+# synthetic inputs (trailing empty reads) and hand-built ones stored with the golden: interior empty reads, single-cell
+# reads, a window without reads (NaN rows), 100 reads, extra feature columns (tests/golden/make_rl_golden.py)
+SYNTH_CASES = ["small", "deep", "dwells", "hot"]
+EDGE_CASES = ["interior_empty", "one_cell", "empty_window", "deep100", "extra_channels"]
+# (k = 17 convolution, LSTM recurrences) on the tensor cores (True) or the fp32 CUDA cores (False)
+PAIRS = {"tc": (True, True), "fp32": (False, False), "tc_lstm32": (True, False), "fp32_lstmtc": (False, True)}
+
+
 def _case(g, name):
     seed, B, P, D, dw, gain = g[name + "_args"]
     sd = rl_oracle.synth_rl_state_dict(int(seed), use_dwells=bool(dw), gain=float(gain))
-    x = rl_oracle.synth_rl_features(int(B), int(P), int(D), use_dwells=bool(dw), seed=100 + int(seed))
+    if name + "_x" in g:
+        x = g[name + "_x"]
+    else:
+        x = rl_oracle.synth_rl_features(int(B), int(P), int(D), use_dwells=bool(dw), seed=100 + int(seed))
     return sd, x, bool(dw), g[name + "_probs"]
 
 
-@pytest.mark.parametrize("name", ["small", "deep", "dwells", "hot"])
+@pytest.mark.parametrize("name", SYNTH_CASES + EDGE_CASES)
 def test_oracle_matches_reference_class(name):
     g = np.load(GOLD)
     sd, x, dw, want = _case(g, name)
     got = rl_oracle.predict(rl_oracle.build(sd, use_dwells=dw), x)
-    assert np.abs(got - want).max() < 2e-6
+    nan = np.isnan(want)
+    assert np.array_equal(np.isnan(got), nan)
+    assert nan.any() == (name == "empty_window")
+    assert np.abs(got[~nan] - want[~nan]).max() < 2e-6
 
 
 def _check(got, want):
@@ -36,37 +50,49 @@ def _check(got, want):
     assert np.array_equal(np.argmax(got, -1)[decided], np.argmax(want, -1)[decided])
 
 
-@pytest.mark.gpu
-@pytest.mark.parametrize("conv", ["tc", "fp32"])
-@pytest.mark.parametrize("name", ["small", "deep", "dwells", "hot"])
-def test_device_matches_reference_class(name, conv):
-    """Both implementations of the k = 17 convolution: tcgen05 implicit GEMM (default) and fp32 CUDA cores."""
+def _model(sd, pair, use_dwells=False):
     from medaka_b200 import read_level
+    m = read_level.LatentSpaceLSTM(use_dwells=use_dwells)
+    m.load_state_dict(sd)
+    m.set_conv(*PAIRS[pair])
+    return m
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("conv", list(PAIRS))
+@pytest.mark.parametrize("name", SYNTH_CASES + EDGE_CASES)
+def test_device_matches_reference_class(name, conv):
+    """Both implementations of the k = 17 convolution (tcgen05 implicit GEMM, fp32 CUDA cores) with both implementations
+    of the LSTM recurrence.  A window without reads is NaN exactly where the reference is; the rest holds the usual bar."""
     g = np.load(GOLD)
     sd, x, dw, want = _case(g, name)
-    m = read_level.LatentSpaceLSTM(use_dwells=dw)
-    m.load_state_dict(sd)
-    m.set_conv(conv == "tc")
-    _check(m.forward_arrays(x), want)
+    m = _model(sd, conv, dw)
+    got = m.forward_arrays(x)
     m.close()
+    nan = np.isnan(want).any(-1)
+    assert np.array_equal(np.isnan(got), np.isnan(want))
+    print("%s/%s: max abs err %.2e" % (name, conv, np.abs(got[~nan] - want[~nan]).max()))
+    _check(got[~nan], want[~nan])
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("conv", ["tc", "fp32"])
-@pytest.mark.parametrize("B,P,D", [(1, 17, 1), (9, 65, 5), (3, 1000, 30), (17, 200, 3), (2, 129, 9)])
+@pytest.mark.parametrize("conv", list(PAIRS))
+@pytest.mark.parametrize("B,P,D", [(1, 17, 1), (9, 65, 5), (3, 1000, 30), (17, 200, 3), (2, 129, 9),
+                                   (3, 1, 4), (4, 8, 2), (2, 16, 8), (3, 127, 4), (2, 128, 8), (2, 256, 2),
+                                   (3, 257, 4), (2, 300, 100)])
 def test_device_matches_oracle_ragged_shapes(B, P, D, conv):
-    """Position counts off the 64-position tile, windows off the 8-window LSTM group, single reads, windows split over
-    several device calls."""
-    from medaka_b200 import read_level
+    """Position counts off the 64- and 128-position convolution tiles and the 16-position pooling tile, windows shorter
+    than the convolution's 8-position halo (P = 1), windows off the LSTM tiles, single reads, 100 reads (25 groups of 4),
+    windows split over several device calls."""
     sd = rl_oracle.synth_rl_state_dict(5)
     x = rl_oracle.synth_rl_features(B, P, D, seed=B * 1000 + P, empty_rows=min(2, D - 1))
     want = rl_oracle.predict(rl_oracle.build(sd), x)
-    m = read_level.LatentSpaceLSTM()
-    m.load_state_dict(sd)
+    m = _model(sd, conv)
     m.max_cells = 40000                      # forces several device calls for the larger shapes
-    m.set_conv(conv == "tc")
-    _check(m.forward_arrays(x), want)
+    got = m.forward_arrays(x)
     m.close()
+    print("%dx%dx%d/%s: max abs err %.2e" % (B, P, D, conv, np.abs(got - want).max()))
+    _check(got, want)
 
 
 @pytest.mark.gpu
